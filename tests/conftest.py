@@ -32,13 +32,6 @@ def oracle(checkers):
 
 
 @pytest.fixture(scope="session")
-def reference(checkers):
-    if not checkers.have_reference("det"):
-        pytest.skip("oracle/_ref not built (no /root/reference and no prebuilt .so)")
-    return checkers.Reference("det")
-
-
-@pytest.fixture(scope="session")
 def product(request):
     """The CUDA product library; built in-tree if missing.  Never falls back to a CPU path."""
     from youtokentome_b200 import _lib

@@ -1,13 +1,14 @@
 """CPU-side checks of the boundary: the C-ABI library loads and exports every symbol that
 include/*.h declares; without a GPU every hot-path entry fails loudly (no CPU fallback); the
 host-only parts of the mirrored surface (model I/O, decode, vocab, id<->subword) agree with the
-reference."""
+reference (its outputs recorded in tests/golden/reference/outputs.json, see _refgolden)."""
 import ctypes as C
 import os
 import re
 
 import pytest
 
+import _refgolden as R
 from _bind import ROOT, tmp_model_path
 from youtokentome_b200 import synth
 
@@ -65,18 +66,23 @@ def test_null_encoder_handle_is_an_error_not_a_crash(product):
     assert b"null encoder handle" in product.yttm_last_error(None)
 
 
-def test_host_surface_matches_reference(product, oracle, reference):
+def test_host_surface_matches_reference(product, oracle):
     """decode / vocab / id_to_subword / subword_to_id / error texts vs the unmodified reference."""
     import youtokentome_b200 as yttm
     m = tmp_model_path()
     train, test, vocab = synth.GOLDEN_TEXTS["russian"]
     oracle.train(train.encode(), m, vocab)
-    bpe, ref = yttm.BPE(m), reference.encoder(m)
-    assert bpe.vocab_size() == ref.vocab_size() == vocab
-    ids = ref.encode([test.encode(), b"ab", b""], bos=True, eos=True)
-    assert bpe.decode(ids) == [ref.decode(s) for s in ids]
+    bpe = yttm.BPE(m)
+    assert bpe.vocab_size() == R.want("abi/host_surface/vocab_size", lambda: R.reference().encoder(m).vocab_size()) == vocab
+    sents = [test.encode(), b"ab", b""]
+    ids = oracle.encoder(m).encode(sents, bos=True, eos=True)
+    assert R.canon(ids) == R.want("abi/host_surface/ids",
+                                  lambda: R.reference().encoder(m).encode(sents, bos=True, eos=True))
+    assert R.canon(bpe.decode(ids)) == R.want("abi/host_surface/decode",
+                                              lambda: [R.reference().encoder(m).decode(s) for s in ids])
     assert bpe.decode(ids, ignore_ids=[2, 3]) != bpe.decode(ids)
-    assert bpe.decode(ids[0]) == [ref.decode(ids[0])]
+    assert R.canon(bpe.decode(ids[0])) == R.want("abi/host_surface/decode0",
+                                                 lambda: [R.reference().encoder(m).decode(ids[0])])
     v = bpe.vocab()
     assert v[:4] == ["<PAD>", "<UNK>", "<BOS>", "<EOS>"] and v[4] == "▁"
     assert all(bpe.subword_to_id(s) == i for i, s in enumerate(v))
@@ -91,27 +97,30 @@ def test_host_surface_matches_reference(product, oracle, reference):
         yttm.BPE("/nonexistent/model")
 
 
-def test_train_argument_errors_match_reference(product, reference):
+def test_train_argument_errors_match_reference(product):
     """check_config (bpe.cpp:1295-1350) runs before any device work: same texts as the reference."""
     import youtokentome_b200 as yttm
     path = tmp_model_path("txt")
     open(path, "w").write("ab ab abc\n")
     cases = [dict(coverage=0.0), dict(coverage=1.5), dict(unk_id=-1), dict(unk_id=50), dict(pad_id=-2),
              dict(bos_id=100), dict(eos_id=77), dict(pad_id=1, unk_id=1)]
-    for kw in cases:
+    def ref_error(args):
+        with pytest.raises(ValueError) as e_ref:
+            R.reference().train_file(path, path + ".m", 20, args["coverage"], 1, args["pad_id"], args["unk_id"],
+                                     args["bos_id"], args["eos_id"])
+        return str(e_ref.value)
+
+    for i, kw in enumerate(cases):
         args = dict(coverage=1.0, pad_id=0, unk_id=1, bos_id=2, eos_id=3)
         args.update(kw)
-        with pytest.raises(ValueError) as e_ref:
-            reference.train_file(path, path + ".m", 20, args["coverage"], 1, args["pad_id"], args["unk_id"],
-                                 args["bos_id"], args["eos_id"])
         with pytest.raises(ValueError) as e_new:
             yttm.BPE.train(path, path + ".m", 20, **args)
-        assert str(e_new.value) == str(e_ref.value)
+        assert str(e_new.value) == R.want("abi/train_errors/%d" % i, lambda: ref_error(args))
     with pytest.raises(ValueError, match="Failed to open file"):
         yttm.BPE.train("/nonexistent/file", path + ".m", 20)
 
 
-def test_cli_host_commands_match_reference_format(product, oracle, reference):
+def test_cli_host_commands_match_reference_format(product, oracle):
     """`yttm vocab [--verbose]` and `yttm decode [--ignore_ids]` (host-only paths, no GPU needed):
     stdout framing of the reference (bpe.cpp:1896-1940, 2016-2028)."""
     import subprocess
@@ -127,9 +136,11 @@ def test_cli_host_commands_match_reference_format(product, oracle, reference):
     verbose = subprocess.run(base + ["vocab", "--model", m, "--verbose"], capture_output=True, text=True, cwd=ROOT,
                              check=True).stdout
     assert "=" in verbose and "+" in verbose
-    ref = reference.encoder(m)
-    ids = ref.encode([test.encode(), b"chrono"], bos=True, eos=True)
+    sents = [test.encode(), b"chrono"]
+    ids = oracle.encoder(m).encode(sents, bos=True, eos=True)
+    assert R.canon(ids) == R.want("abi/cli/ids", lambda: R.reference().encoder(m).encode(sents, bos=True, eos=True))
     stdin = "\n".join(" ".join(map(str, s)) for s in ids) + "\n"
     dec = subprocess.run(base + ["decode", "--model", m, "--ignore_ids", "2,3"], input=stdin, capture_output=True,
                          text=True, cwd=ROOT, check=True).stdout
-    assert dec.split("\n")[:-1] == [ref.decode([i for i in s if i not in (2, 3)]) for s in ids]
+    assert R.canon(dec.split("\n")[:-1]) == R.want(
+        "abi/cli/decode", lambda: [R.reference().encoder(m).decode([i for i in s if i not in (2, 3)]) for s in ids])

@@ -116,14 +116,14 @@ def test_host_alphabet_and_model_writer_match_oracle(oracle, cov):
 @pytest.mark.parametrize("special", [(0, 1, 2, 3), (-1, 0, -1, 5)])
 def test_model_writer_is_byte_identical_to_the_reference(special):
     """write_model (rank 0 of train_distributed) writes the very bytes the reference's BPEState::dump does,
-    char2id lines in flat_hash_map order included: feed it the reference's own result un-renamed."""
+    char2id lines in flat_hash_map order included (the reference's file recorded by its SHA-256, see _refgolden):
+    feed it the trained model un-renamed."""
     import _bind
-    if not _bind.have_reference("det"):
-        pytest.skip("oracle/_ref not built")
+    import _refgolden as R
     pad, unk, bos, eos = special
     text = _cases.zipf().text(60_000)
-    m = tmp_model_path("refw")
-    _bind.Reference("det").train(text, m, 900, 1.0, n_threads=1, pad=pad, unk=unk, bos=bos, eos=eos)
+    m = tmp_model_path("orcw")
+    _bind.Oracle().train(text, m, 900, 1.0, pad=pad, unk=unk, bos=bos, eos=eos)
     c2i, rules, _ = read_model(m)
     # undo rename_tokens: final ids -> internal ids (specials first, then the rest ascending)
     taken = {s for s in special if s != -1}
@@ -133,5 +133,5 @@ def test_model_writer_is_byte_identical_to_the_reference(special):
     internal = np.asarray([[back[x], back[y], back[z]] for x, y, z in rules], dtype=np.uint32).reshape(-1, 3)
     out = tmp_model_path("oursw")
     D.write_model(out, char2id, internal, special, 900)
-    with open(m, "rb") as a, open(out, "rb") as b:
-        assert a.read() == b.read()
+    assert R.file_sha256(out) == R.want("distributed/model_writer/%d_%d_%d_%d" % special, lambda: R.file_sha256(
+        R.train(text, 900, 1.0, pad=pad, unk=unk, bos=bos, eos=eos)))

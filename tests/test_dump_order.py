@@ -1,7 +1,7 @@
 """Byte-identical model dump (SURVEY.md §8f-4): the char2id lines of a model written by the reference
 come in ska::flat_hash_map slot order (utils.cpp:57-59).  `yttm_api_dump_order` replays that order
 from the insertion sequence alone; checked here against model files the UNMODIFIED reference writes
-(oracle/_ref, DETERMINISTIC_QUEUE build) — CPU only, no GPU needed."""
+(DETERMINISTIC_QUEUE build, recorded in tests/golden/reference/outputs.json, see _refgolden) — CPU only, no GPU needed."""
 import ctypes as C
 import os
 
@@ -9,10 +9,9 @@ import numpy as np
 import pytest
 
 import _bind
+import _refgolden as R
 from _cases import dirty_zipf_text, stress_case, zipf
 from youtokentome_b200 import _lib, synth
-
-pytestmark = pytest.mark.skipif(not _bind.have_reference("det"), reason="oracle/_ref not built")
 
 
 def file_order(path):
@@ -32,12 +31,14 @@ def replay(char2id):
     return out.tolist()
 
 
-def check(text, vocab, coverage=1.0, **special):
+def check(key, text, vocab, coverage=1.0, **special):
+    """replay() of the char2id of this training == the code point order of the reference's model file."""
     path = _bind.tmp_model_path("dumporder")
     try:
-        _bind.Reference("det").train(text, path, vocab, coverage, n_threads=1, **special)
-        order, c2i = file_order(path)
-        assert replay(c2i) == order
+        _bind.Oracle().train(text, path, vocab, coverage, **special)
+        order = replay(_bind.read_model(path)[0])
+        assert R.canon(order) == R.want("dump_order/" + key,
+                                        lambda: file_order(R.train(text, vocab, coverage, **special))[0])
         return len(order)
     finally:
         if os.path.exists(path):
@@ -47,24 +48,24 @@ def check(text, vocab, coverage=1.0, **special):
 @pytest.mark.parametrize("seed", range(12))
 def test_stress_alphabets(seed):
     text, vocab, cov, _ = stress_case(seed)
-    check(text, vocab, cov)
+    check("stress/%d" % seed, text, vocab, cov)
 
 
 def test_readme_alphabet():
-    assert check(synth.readme_corpus(200), 300) == 5
+    assert check("readme", synth.readme_corpus(200), 300) == 5
 
 
 def test_multiscript_alphabets():
     # thousands of code points: several doublings of the table, robin-hood displacement chains
-    n = check(zipf().text(400_000), 4000)
+    n = check("multiscript", zipf().text(400_000), 4000)
     assert n > 300
-    check(dirty_zipf_text(), 3500, 0.999)
+    check("dirty", dirty_zipf_text(), 3500, 0.999)
 
 
 def test_coverage_and_special_ids():
     t = zipf().text(150_000)
-    check(t, 3500, 0.98)
-    check(t, 3500, 1.0, pad=-1, bos=-1, eos=7, unk=0)
+    check("coverage", t, 3500, 0.98)
+    check("special_ids", t, 3500, 1.0, pad=-1, bos=-1, eos=7, unk=0)
 
 
 def test_wide_code_point_range():
@@ -73,12 +74,12 @@ def test_wide_code_point_range():
     cps = np.concatenate([rng.integers(0x21, 0x7f, 40), rng.integers(0x400, 0x500, 60), rng.integers(0x4e00, 0x9fff, 700),
                           rng.integers(0x1f300, 0x1f700, 200)])
     words = ["".join(chr(int(c)) for c in rng.choice(cps, int(rng.integers(1, 7)))) for _ in range(6000)]
-    check(" ".join(words).encode(), len(set(cps.tolist())) + 50)
+    check("wide_range", " ".join(words).encode(), len(set(cps.tolist())) + 50)
 
 
 # ---- the replay against the reference's own container on arbitrary key sets ---------------------
 def ref_order(keys):
-    lib = _bind.Reference("det").lib
+    lib = R.reference().lib
     lib.ref_char2id_order.restype = C.c_int
     lib.ref_char2id_order.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p]
     keys = np.ascontiguousarray(keys, dtype=np.uint32)
@@ -104,7 +105,7 @@ def test_random_keys_match_the_reference_container(n):
         keys = rng.permutation(np.unique(rng.integers(0, hi, n + 8)))[:n]
         if len(keys) < n:
             continue
-        assert our_order(keys) == ref_order(keys)
+        assert R.canon(our_order(keys)) == R.want("dump_order/random/%d/%x" % (n, hi), lambda: ref_order(keys))
 
 
 def test_clustered_home_slots_force_regrowth():
@@ -117,26 +118,25 @@ def test_clustered_home_slots_force_regrowth():
     for n in (6, 12, 40, 200):
         clustered = cand[top == top[0]][:n]                  # same home slot in every table up to 4096 buckets
         mixed = np.concatenate([clustered, cand[:n]])
-        for keys in (clustered, rng.permutation(np.unique(mixed))):
-            assert our_order(keys) == ref_order(keys)
+        for j, keys in enumerate((clustered, rng.permutation(np.unique(mixed)))):
+            assert R.canon(our_order(keys)) == R.want("dump_order/clustered/%d/%d" % (n, j), lambda: ref_order(keys))
 
 
 def test_sequential_and_strided_keys():
-    for keys in (np.arange(0, 3000), np.arange(0, 300000, 97), np.arange(2 ** 32 - 2000, 2 ** 32 - 1),
-                 (np.arange(1, 2000, dtype=np.uint64) * 2654435769 % 2 ** 32)):
-        assert our_order(keys) == ref_order(keys)
+    for j, keys in enumerate((np.arange(0, 3000), np.arange(0, 300000, 97), np.arange(2 ** 32 - 2000, 2 ** 32 - 1),
+                              (np.arange(1, 2000, dtype=np.uint64) * 2654435769 % 2 ** 32))):
+        assert R.canon(our_order(keys)) == R.want("dump_order/sequential/%d" % j, lambda: ref_order(keys))
 
 
 # ---- the product's BPEState::dump writes the reference's bytes -----------------------------------
-def _redump_equals(path):
+def _redump_sha256(path):
     L = _lib.lib()
     L.yttm_api_redump.restype = C.c_int
     L.yttm_api_redump.argtypes = [C.c_char_p, C.c_char_p]
     out = path + ".redump"
     try:
         assert L.yttm_api_redump(path.encode(), out.encode()) == 0
-        with open(path, "rb") as a, open(out, "rb") as b:
-            assert a.read() == b.read()
+        return R.file_sha256(out)
     finally:
         if os.path.exists(out):
             os.remove(out)
@@ -151,10 +151,11 @@ def test_product_dump_is_byte_identical_to_the_reference_file(case):
         "stress3": stress_case(3)[:3] + ({},),
         "special_ids": (zipf().text(100_000), 2000, 1.0, dict(pad=-1, bos=-1, eos=5, unk=0)),
     }[case]
-    path = _bind.tmp_model_path("refdump")
+    path = _bind.tmp_model_path("orcdump")
     try:
-        _bind.Reference("det").train(text, path, vocab, cov, n_threads=1, **special)
-        _redump_equals(path)
+        _bind.Oracle().train(text, path, vocab, cov, **special)
+        assert _redump_sha256(path) == R.want("dump_order/redump/" + case,
+                                              lambda: R.file_sha256(R.train(text, vocab, cov, **special)))
     finally:
         if os.path.exists(path):
             os.remove(path)

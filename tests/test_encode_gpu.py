@@ -6,7 +6,8 @@ import numpy as np
 import pytest
 
 import _cases
-from _bind import _pack, tmp_model_path
+import _refgolden as R
+from _bind import _pack, read_model, tmp_model_path
 from _gpu import GpuEncoder, gpu_train
 from youtokentome_b200 import synth
 
@@ -81,14 +82,13 @@ def test_dropout_matches_oracle_stream(product, oracle, p):
     assert sum(map(len, a)) >= sum(map(len, base))
 
 
-def test_dropout_distribution_vs_reference(product, checkers, oracle):
-    """mean tokens / sentence at p = 0.1 within 2 % of the reference's own DropoutQueue."""
-    if not checkers.have_reference("det"):
-        pytest.skip("oracle/_ref absent")
+def test_dropout_distribution_vs_reference(product, oracle):
+    """mean tokens / sentence at p = 0.1 within 2 % of the reference's own DropoutQueue (its total recorded, see
+    _refgolden)."""
     m = _model(oracle, _cases.dirty_zipf_text(), 1500)
     sents = _cases.zipf_sentences(3000)
-    ref = checkers.Reference("det").encoder(m, n_threads=1)
-    r = sum(map(len, ref.encode(sents, dropout=0.1)))
+    r = R.want("encode_gpu/dropout_total_ids",
+               lambda: sum(map(len, R.reference().encoder(m, n_threads=1).encode(sents, dropout=0.1))))
     g = sum(map(len, GpuEncoder(m).encode(sents, dropout=0.1, seed=99)))
     assert abs(g - r) / r < 0.02
 
@@ -163,18 +163,18 @@ def test_python_api_roundtrip(product, tmp_path):
     assert pickle.loads(pickle.dumps(bpe)).encode(test_lines[:5]) == bpe.encode(test_lines[:5])
 
 
-def test_config2_shape_vs_reference(product, checkers):
+def test_config2_shape_vs_reference(product):
     """BASELINE config 2 shape at 1/20 scale: 50k x 128-byte Zipf sentences, vocab 8000 model
-    trained by the reference; ids identical to the reference (8 threads)."""
-    if not checkers.have_reference("det"):
-        pytest.skip("oracle/_ref absent")
+    trained on the GPU == the reference's; ids identical to the reference (8 threads; recorded, see _refgolden)."""
     zc = synth.ZipfCorpus(n_words=50_000, seed=11)
-    ref = checkers.Reference("det")
-    m = tmp_model_path("ref")
-    ref.train(zc.text(6_000_000), m, 8000, 1.0, n_threads=8)
+    text = zc.text(6_000_000)
     sents = zc.sentences(50_000, 128, seed=77)
-    want = ref.encoder(m, n_threads=8).encode(sents)
-    assert GpuEncoder(m).encode(sents) == want
+    want_model = R.want("encode_gpu/config2/model", lambda: R.model(text, 8000, 1.0, threads=8))
+    want_ids = R.want("encode_gpu/config2/ids",
+                      lambda: R.reference().encoder(R.train(text, 8000, 1.0, threads=8), n_threads=8).encode(sents))
+    m = gpu_train(text, 8000, 1.0)
+    assert R.canon(read_model(m)) == want_model
+    assert R.canon(GpuEncoder(m).encode(sents)) == want_ids
 
 
 def test_chunked_h2d_pipeline(product, oracle, monkeypatch):

@@ -1,8 +1,9 @@
 """The reference's OWN stress test (tests/unit_tests/stress_test.cpp: learn_bpe_slow / decode_slow specs, seeds,
-manual case, batch == single) compiled UNMODIFIED — fed to g++ on stdin from /root/reference, never copied — against
-this repo's drop-in headers (include/compat) and run against the product's kernels under the SIMT emulator
-(tests/emul/simt; test harness only).  The same source linked with the real libyttm_b200.so is built by oracle/Makefile
-into oracle/_ref/ref_stress_b200 and run on the B200 by tests/test_zz_reference_stress_gpu.py."""
+manual case, batch == single) run against the product's kernels under the SIMT emulator (tests/emul/simt; test harness
+only).  The binary is oracle/_ref/ref_stress_b200, which build() compiles (oracle/Makefile) from the unmodified source
+against this repo's drop-in headers (include/compat) where the reference's sources are present; it is linked with
+libyttm_b200.so, and here the emulator build takes that name on LD_LIBRARY_PATH, which its RUNPATH gives way to.
+tests/test_zz_reference_stress_gpu.py runs the same binary with the real library on the B200."""
 import os
 import subprocess
 
@@ -10,28 +11,23 @@ import pytest
 
 from _bind import ROOT
 
-REF_TEST = "/root/reference/tests/unit_tests/stress_test.cpp"
-pytestmark = pytest.mark.skipif(not os.path.exists(REF_TEST), reason="needs /root/reference (absent on the GPU box)")
+BIN = os.path.join(ROOT, "oracle", "_ref", "ref_stress_b200")
+pytestmark = pytest.mark.skipif(not os.path.exists(BIN), reason="oracle/_ref/ref_stress_b200 not built")
 
 
 @pytest.fixture(scope="module")
-def stress_binary():
+def emulated_lib_dir(tmp_path_factory):
+    """A directory where libyttm_b200.so is the emulator build of the kernels."""
     from _emu import emu_lib
     emu_lib()  # builds tests/emul/simt/_gen/libyttm_emu.so
-    gen = os.path.join(ROOT, "tests", "emul", "simt", "_gen")
-    out = os.path.join(gen, "ref_stress_emu")
-    lib = os.path.join(gen, "libyttm_emu.so")
-    if not os.path.exists(out) or os.path.getmtime(out) < os.path.getmtime(lib):
-        with open(REF_TEST, "rb") as src:
-            subprocess.run(["/usr/bin/g++", "-std=c++17", "-O1", "-pthread", "-w", "-x", "c++", "-", "-o", out, "-L" + gen,
-                            "-lyttm_emu", "-Wl,-rpath," + gen], stdin=src, check=True,
-                           cwd=os.path.join(ROOT, "include", "compat", "tests", "unit_tests"))
-    return out
+    d = tmp_path_factory.mktemp("emulated_lib")
+    os.symlink(os.path.join(ROOT, "tests", "emul", "simt", "_gen", "libyttm_emu.so"), d / "libyttm_b200.so")
+    return str(d)
 
 
 @pytest.mark.parametrize("args", [["manual"], ["base", "60"], ["parallel", "6"]])
-def test_reference_stress_test_passes_on_the_emulated_kernels(stress_binary, tmp_path, args):
-    env = dict(os.environ, YT_EMU_SMS="2")
-    r = subprocess.run([stress_binary] + args, cwd=tmp_path, env=env, stdout=subprocess.DEVNULL, stderr=subprocess.PIPE,
+def test_reference_stress_test_passes_on_the_emulated_kernels(emulated_lib_dir, tmp_path, args):
+    env = dict(os.environ, YT_EMU_SMS="2", LD_LIBRARY_PATH=emulated_lib_dir)
+    r = subprocess.run([BIN] + args, cwd=tmp_path, env=env, stdout=subprocess.DEVNULL, stderr=subprocess.PIPE,
                        timeout=900)
     assert r.returncode == 0, r.stderr.decode(errors="replace")[-2000:]

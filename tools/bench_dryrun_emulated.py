@@ -6,6 +6,7 @@ through distributed.train_distributed with their reference parity checks, the sc
 with its oracle check, the CPU baselines with the id comparison and the ONE JSON line.
 The numbers mean nothing; the point is that a slip in bench.py shows up here and not on the driver's GPU box.
     python tools/bench_dryrun_emulated.py [extra bench.py flags]  > line.json"""
+import ctypes as C
 import os
 import sys
 
@@ -15,6 +16,7 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 os.environ.setdefault("YT_EMU_SMS", "2")
 os.environ.setdefault("YTTM_BENCH_CACHE", "/tmp/yttm_b200_bench_dryrun_cache")
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 from _emu import emu_lib  # noqa: E402
 from youtokentome_b200 import _lib  # noqa: E402
@@ -42,5 +44,8 @@ class _NoClocks:
 
 
 bench.ClockSampler = _NoClocks
+# the emulator's "device" memory is host memory
+bench.device_array = lambda ptr, n, typestr: np.frombuffer((C.c_char * (n * np.dtype(typestr).itemsize)).from_address(ptr),
+                                                           dtype=typestr).copy()
 sys.argv = ["bench.py", "--steps", "2", "--warmup", "3", "--scan-tokens", "131072"] + sys.argv[1:]
 bench.main()
